@@ -2,12 +2,14 @@
 """bench.py -- images/sec of the CRNN forward + CTC loss hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c2tf32|c2shape|c1shape] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = conv stack -> BiLSTM -> logits -> CTC loss (+gradient, as warp-ctc's forward op computes it)
 -> mean + L2, over one synthetic batch.  Default workload = BASELINE.json configs[2] (1xB200 bf16 tcgen05 path,
 batch 1024, 32x256): the configuration the north-star targets are quoted on; under torchrun every rank runs the
 same per-GPU batch (weak scaling, batch-sharded, no data-path collective for the forward).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR: rank 0 also writes what the last timed step returned to its caller
+(logits, ctc_costs, ctc_grad, loss) as DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -197,7 +199,10 @@ def main():
     ap.add_argument("--sync-bn-forward", action="store_true", help="N>1: global-batch BN also in the forward-only metric (default: replicas)")
     ap.add_argument("--bucket-mb", type=float, default=8.0, help="N>1: merge announced gradient ranges until this many MB are ready")
     ap.add_argument("--sm-reserve", type=int, default=8, help="N>1 with overlap: SMs the persistent backward kernels leave to the collectives")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -293,6 +298,11 @@ def main():
         loss = model.total_loss(costs)
     e1.record()
     sync_all()
+    if args.dump_outputs and rank == 0:
+        # read before the sections below reuse these buffers: ~33 MB at c3, all f32
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("logits", logits), ("ctc_costs", costs), ("ctc_grad", grad), ("loss", loss)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
     ms_total = e0.elapsed_time(e1)
     loss_val = float(loss.item())
     nst = model.lib.crnn_profile_num_stages()

@@ -42,8 +42,7 @@ def gen_rand(rng=random, min_len=None, max_len=None):
 def _font_path():
     if os.environ.get("CRNN_FONT", "") == "default":      # force Pillow's embedded scalable font (identical on every box)
         return None
-    for p in (cfg.FONT, os.path.join(cfg.ROOT_DIR, cfg.FONT), os.path.join(os.path.dirname(os.path.abspath(__file__)), "Ubuntu-M.ttf"),
-              os.path.join("/root/reference", cfg.FONT)):
+    for p in (cfg.FONT, os.path.join(cfg.ROOT_DIR, cfg.FONT), os.path.join(os.path.dirname(os.path.abspath(__file__)), "Ubuntu-M.ttf")):
         if os.path.exists(p):
             return p
     for p in ("/usr/share/fonts/truetype/dejavu/DejaVuSans-Bold.ttf", "/usr/share/fonts/truetype/dejavu/DejaVuSans.ttf"):

@@ -539,6 +539,14 @@ def test_bench_reference_arm_prints_the_contract_line_and_ours_refuses_without_a
         assert p.returncode != 0 and "no CPU fallback" in (p.stderr + p.stdout)
 
 
+def test_bench_refuses_fewer_than_one_timed_step():
+    import subprocess
+    import sys
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0", "--dump-outputs", "unused"],
+                       capture_output=True, text=True, timeout=600)
+    assert p.returncode == 2 and "--steps must be at least 1" in p.stderr
+
+
 def build_c_abi_smoke(tmp_path):
     """gcc -std=c99 tests/c_abi/abi_smoke.c against include/crnn_ctc.h and the in-tree libcrnnctc.so; returns the binary's path."""
     import subprocess

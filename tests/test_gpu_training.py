@@ -182,7 +182,7 @@ def test_eval_solver_walks_a_directory_like_the_reference(tmp_path, capsys):
     assert "total acc:" in out and "cost time:" in out and "Restoring from" in out
 
 
-def test_training_on_fresh_renders_learns_to_read():
+def test_training_on_fresh_renders_learns_to_read(tmp_path):
     """VERDICT r1 weak #4 ('training does not demonstrably learn'): the reference-shaped solver on FRESH renders every step (lines of
     4-6 characters, batch 64, lr 1e-4: lstm/lstm.yml + lib/lstm/utils/gen.py:69-110), fed by the page-locked PrefetchFeeder, from
     the reference initialisers.  4 000 iterations (~10 s on a B200) reach > 99 % held-out exact match in the committed run
@@ -206,7 +206,7 @@ def test_training_on_fresh_renders_learns_to_read():
     try:
         net = get_network("LSTM_train")
         with Session(device=DEV) as sess:
-            sw = T.SolverWrapper(sess, net, None, None, "/tmp/crnn_learn_out", "/tmp/crnn_learn_log")
+            sw = T.SolverWrapper(sess, net, None, None, str(tmp_path / "out"), str(tmp_path / "log"))
             hist = sw.train_model(sess, 4001, restore=False, train_gen=feeder, val_gen=iter(held))
             assert len(hist) == 4000 and np.mean(hist[-200:]) < 0.15 * np.mean(hist[:200]), (np.mean(hist[:200]), np.mean(hist[-200:]))
             _, dec_h = net.build_loss()
